@@ -71,7 +71,11 @@ def main():
     ap.add_argument("--min-seconds", type=float, default=2.0, help="lower bound on the timed region (msgs_per_step is sized for it)")
     ap.add_argument("--msgs-per-step", type=int, default=0, help="0 = calibrate")
     ap.add_argument("--extras", type=int, default=1, help="also run baselines' siblings: ring, fused pack, small messages, GEMM, mock NIC")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last step delivered (rank 0) as DIR/<name>.npy, to compare two builds")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return reference_arm()
     quiet_stdout()
@@ -89,7 +93,7 @@ def main():
     if world != args.gpus and world > 1:
         args.gpus = world
     warmup = max(args.warmup, 3)
-    steps = max(args.steps, 1)
+    steps = args.steps
     if not torch.cuda.is_available():
         # the GPU-initiated path has no CPU fallback by design: say so in one line instead of a traceback
         if rank == 0:
@@ -220,6 +224,8 @@ def main():
     engine_off()
     # byte verification: every destination slot equals its source slot
     n_bad = sum(ops.compare(src[i * msg:(i + 1) * msg], dst[i * msg:(i + 1) * msg]) for i in range(nslots))
+    if args.dump_outputs and rank == 0:                               # before the baselines below overwrite dst
+        dump_outputs(args.dump_outputs, dst, msg, nslots, last, mps)
 
     # ---------------- baselines in the same process, same buffers, same wire
     base = {}
@@ -539,6 +545,22 @@ def main():
         dist.destroy_process_group()
     ctx.close()
     return 0
+
+
+def dump_outputs(path, dst, msg, nslots, last, mps):
+    """What the last timed step delivered, as float arrays under ``path``: a fixed, seeded sample of 4 Mi destination bytes
+    (16 MB), the exact byte sum of every destination slot, and the step's completion status.  The source bytes are
+    seeded, so with the same arguments two builds must write the same files.  The message count per step follows the
+    calibration unless ``--msgs-per-step`` fixes it, so the status records the completed fraction, not the count."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    n = msg * nslots
+    idx = torch.randint(0, n, (min(n, 1 << 22),), generator=torch.Generator().manual_seed(0)).sort().values
+    np.save(os.path.join(path, "dst_bytes_sample.npy"), dst[idx.to(dst.device)].float().cpu().numpy())
+    sums = [float(dst[s * msg:(s + 1) * msg].sum(dtype=torch.int64)) for s in range(nslots)]
+    np.save(os.path.join(path, "dst_slot_byte_sums.npy"), np.array(sums, dtype=np.float64))
+    np.save(os.path.join(path, "last_step_status.npy"), np.array([float(last.ok), sum(last.done) / mps], dtype=np.float64))
 
 
 def mock_nic_extra(rn, ops, W, N, C, device, src, dst):

@@ -33,6 +33,7 @@
 #include <unistd.h>
 
 #include <atomic>
+#include <map>
 #include <mutex>
 #include <thread>
 #include <vector>
@@ -146,7 +147,29 @@ struct QpH {
   uint64_t next_wr_id = 1;
   bool raw_owned = false;     // queues handed to the GPU: host posting would fight over the producer index
   int proxy_slot = -1;
+  std::vector<uint64_t> host_regs;   // pages of g_host_regs this QP holds (rn_verbs_map_qp_to_gpu)
 };
+
+// Host ranges this library cudaHostRegister()ed to map a QP's queues into the GPU, keyed by first page, with the
+// number of QPs using each (CQs and UAR pages can be shared by QPs).  The memory belongs to the provider, which
+// frees it when the QP / CQ is destroyed: the registration must go first, or it stays on freed heap pages and a
+// later queue allocated across them fails to map (cudaHostRegister reports "already registered" for a range whose
+// first page has no device pointer).
+std::mutex g_host_regs_mu;
+std::map<uint64_t, int> g_host_regs;
+
+void host_regs_release(std::vector<uint64_t>& pages) {
+  std::lock_guard<std::mutex> g(g_host_regs_mu);
+  for (uint64_t p : pages) {
+    auto it = g_host_regs.find(p);
+    if (it == g_host_regs.end() || --it->second > 0) continue;
+    g_host_regs.erase(it);
+    cudaHostUnregister((void*)p);
+    cudaGetLastError();
+  }
+  pages.clear();
+}
+
 struct MrH { Dev* dev; ibv_mr* mr; int mode; };
 
 // ---------------------------------------------------------------- CPU doorbell proxy
@@ -367,6 +390,7 @@ RN_API void* rn_verbs_create_qp(void* dev, void* scq, void* rcq, uint32_t sq_dep
 RN_API int rn_verbs_destroy_qp(void* qp) {
   QpH* q = (QpH*)qp;
   proxy_detach(q->proxy_slot);
+  host_regs_release(q->host_regs);
   int rc = api().destroy_qp(q->qp);
   delete q;
   return rc ? -rc : 0;
@@ -604,7 +628,15 @@ RN_API int rn_verbs_map_qp_to_gpu(void* qp, RnGpuQp* out) {
   auto map = [&](uint64_t host, size_t bytes, unsigned flags, uint64_t* dev, bool quiet) -> int {
     const uint64_t page = host & ~4095ull;
     const size_t len = ((host + bytes + 4095) & ~4095ull) - page;
-    cudaError_t e = cudaHostRegister((void*)page, len, flags);
+    cudaError_t e;
+    {
+      std::lock_guard<std::mutex> g(g_host_regs_mu);
+      e = cudaHostRegister((void*)page, len, flags);
+      if (e == cudaSuccess || (e == cudaErrorHostMemoryAlreadyRegistered && g_host_regs.count(page))) {
+        ++g_host_regs[page];
+        q->host_regs.push_back(page);
+      }
+    }
     if (e != cudaSuccess && e != cudaErrorHostMemoryAlreadyRegistered) {
       cudaGetLastError();
       if (!quiet) why(-5, "cudaHostRegister(0x%llx, %zu, 0x%x): %s", (unsigned long long)page, len, flags, cudaGetErrorString(e));

@@ -59,3 +59,29 @@ def ctx():
     c = rn.Context(device=0)
     yield c
     c.close()
+
+
+@pytest.fixture(scope="session")
+def dmabuf_export_error():
+    """None when the GPU driver exports device memory as a dma-buf, else the CUresult it refused with.  The device
+    attribute is not enough: a paravirtualised driver (gVisor's nvproxy) reports CU_DEVICE_ATTRIBUTE_DMA_BUF_SUPPORTED
+    and refuses every export."""
+    import ctypes as C
+    import torch
+    from rocnrdma_b200 import _native as N
+    lib = N.load()
+    t = torch.empty(4 << 20, dtype=torch.uint8, device="cuda:0")
+    lo = (t.data_ptr() + 65535) & ~65535
+    lib.rn_set_device(0)
+    cu = C.c_int(0)
+    fd = lib.rn_dmabuf_export(lo, 1 << 20, C.byref(cu))
+    if fd >= 0:
+        lib.rn_dmabuf_close(fd)
+        return None
+    return cu.value
+
+
+@pytest.fixture
+def needs_dmabuf_export(dmabuf_export_error):
+    if dmabuf_export_error is not None:
+        pytest.skip(f"this GPU driver refuses dma-buf export of device memory (CUresult {dmabuf_export_error})")

@@ -3,7 +3,7 @@
 // for their own GPU-initiated mlx5 posting).  tests/test_wire_format.py compares the native encoder with a Python
 // mirror written by the same hand as the encoder; this file is the outside reference the verdict asked for: if a field
 // offset, a segment size, an opcode or a flag of ours disagreed with theirs, it would not compile.
-// Built with -fsyntax-only by tests/test_wire_crosscheck.py (header path discovered at run time).
+// Built with -fsyntax-only by tests/test_wire_crosscheck.py (header: the copy in tests/golden).
 #include <stddef.h>
 #include <stdint.h>
 

@@ -27,7 +27,7 @@ def test_twin_classifies_addresses_and_page_size():
     be.close()
 
 
-def test_twin_pin_multi_pin_and_cpu_window():
+def test_twin_pin_multi_pin_and_cpu_window(needs_dmabuf_export):
     be = H.UserBackend()
     t = _buf(8 * PAGE)
     va = t.data_ptr()
@@ -52,7 +52,7 @@ def test_twin_pin_multi_pin_and_cpu_window():
     assert be.close() == 1                               # close-with-leaks releases the rest
 
 
-def test_twin_cpu_mapping_of_the_pin_is_attempted_and_reported():
+def test_twin_cpu_mapping_of_the_pin_is_attempted_and_reported(needs_dmabuf_export):
     """The kernel harness maps the pinned pages into the caller (reference: tests/amdp2ptest.c:336-395).  From userspace the
     only handle on a pin is its dma-buf: mmap() of that fd is the same window where the exporter implements it.  Either it
     maps -- then peek / poke are CPU accesses through the BAR and must agree with the GPU's view -- or the attempt fails
@@ -85,7 +85,7 @@ def test_twin_rejects_misaligned_and_host_ranges():
     be.close()
 
 
-def test_reg_mr_dmabuf_mode_holds_a_pin(ctx):
+def test_reg_mr_dmabuf_mode_holds_a_pin(needs_dmabuf_export, ctx):
     import os
     t = _buf(1 << 20)
     mr = ctx.reg_mr(t, nbytes=1 << 20, mode="dmabuf")

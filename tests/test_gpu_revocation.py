@@ -32,7 +32,9 @@ def test_tensor_registration_pins_its_storage(ctx):
 
 
 @pytest.mark.parametrize("mode", ["direct", "dmabuf"])
-def test_free_under_a_live_registration_revokes_it(ctx, mode):
+def test_free_under_a_live_registration_revokes_it(request, ctx, mode):
+    if mode == "dmabuf":
+        request.getfixturevalue("needs_dmabuf_export")
     src = torch.full((4096,), 3, dtype=torch.uint8, device="cuda:0")
     ms = ctx.reg_mr(src)
     x = _victim()

@@ -31,12 +31,15 @@ def _bufs(n):
 
 
 @pytest.mark.parametrize("mode", ["peermem", "dmabuf", "auto"])
-def test_host_posted_write_on_hbm_mrs(vctx, mode):
-    """BASELINE config 2 shape: cudaMalloc HBM registered with the HCA, host-posted RDMA write, CPU-polled CQ."""
+def test_host_posted_write_on_hbm_mrs(request, dmabuf_export_error, vctx, mode):
+    """BASELINE config 2 shape: cudaMalloc HBM registered with the HCA, host-posted RDMA write, CPU-polled CQ.  ``auto``
+    takes the dma-buf where the driver exports one and falls back to the peer-memory client where it does not."""
+    if mode == "dmabuf":
+        request.getfixturevalue("needs_dmabuf_export")
     n = 1 << 20
     src, dst = _bufs(n)
     ms, md = vctx.reg_mr(src, mode=mode), vctx.reg_mr(dst, mode=mode)
-    assert ms.mode == ("dmabuf" if mode in ("dmabuf", "auto") else "peermem")
+    assert ms.mode == ("dmabuf" if mode == "dmabuf" or (mode == "auto" and dmabuf_export_error is None) else "peermem")
     assert (ms.dmabuf_fd >= 0) == (ms.mode == "dmabuf")
     qp = vctx.loopback_qp(depth=16, mem=W.MEM_HOST_PINNED)
     assert not qp.on_gpu
